@@ -66,14 +66,12 @@ DT2 = 0.025 ** 2
 
 def build_scene(args):
     """N=1 workload = the configuration the metric is quoted on: BASELINE config C5, the 1M-tet ball pile.
-    scene "c5"  : as specified in BASELINE.md / SURVEY 8(d) -- 146 x input/tetMeshes/sphere1K.msh on a jittered FCC lattice (needs the
-                  assets/_ref cache that __graft_entry__.build() makes from the reference's meshes);
+    scene "c5"  : as specified in BASELINE.md / SURVEY 8(d) -- 146 x input/tetMeshes/sphere1K.msh (stored as tests/golden/sphere1K.npz)
+                  on a jittered FCC lattice;
     scene "pile": round 1's synthetic pile (167 rounded L6 balls of 6000 tets stacked in columns) -- kept as a second line; it has
                   ~4x the active pairs of C5 because its balls touch over flat poles."""
-    from ipc_b200 import msh, scenes
+    from ipc_b200 import scenes
     scene = getattr(args, "scene", "c5")
-    if scene == "c5" and not msh.have_asset("sphere1K"):
-        scene = "pile"
     if scene == "c5":
         n_balls = max(1, int(round(args.tets / 6851)))
         m, info = scenes.sphere_pile_fcc(n_balls, seed=5, energy=0)
@@ -215,6 +213,28 @@ KAPPA = 1e8
 TI_TOL = 1e-6
 
 
+DUMP_MAX_VALUES = {"gradient": 1 << 21, "csr_values": 1 << 22}  # --dump-outputs stays under 48 MB of float64 at any --tets
+
+
+def dump_outputs(path, ctx, it, n_grad, own0, own1):
+    """--dump-outputs: what a caller of the timed path receives after its last step, as float64 arrays.
+      gradient.npy     the gradient (elastic + barrier), summed over the ranks
+      csr_values.npy   the Hessian's CSR values (elastic + mass + barrier) of the rows this rank owns (all of them on one rank)
+      energy.npy       [elastic, barrier] energies of the iteration record
+      step_bound.npy   [inversion, partial CCD, swept grid, full CCD, final] step bounds of the iteration record
+    An array longer than DUMP_MAX_VALUES[name] is written as its values at a fixed sample of positions (seed 0, increasing order)."""
+    from ipc_b200 import lib as L
+    os.makedirs(path, exist_ok=True)
+    out = {"gradient": ctx.download(L.BUF_GRADIENT, n_grad), "csr_values": ctx.download(L.BUF_CSR_VALUES, own1)[own0:],
+           "energy": np.array([it.energy_elastic, it.energy_barrier]),
+           "step_bound": np.array([it.alpha_inversion, it.alpha_partial_ccd, it.alpha_swept_grid, it.alpha_full_ccd, it.alpha])}
+    for name, a in out.items():
+        cap = DUMP_MAX_VALUES.get(name, a.size)
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -227,6 +247,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run parity check against the oracle (rank 0, before the warm-up)")
     ap.add_argument("--eager", action="store_true", help="enqueue every launch of the timed steps one by one instead of replaying the captured CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (rank 0, see dump_outputs)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -393,6 +414,8 @@ def main():
     launches = ctx.launch_count() - n0
     ms_step = ms_total / args.steps
     it = stats["it"]
+    if rank == 0 and args.dump_outputs:  # before the passes below overwrite the device buffers
+        dump_outputs(args.dump_outputs, ctx, it, 3 * m.nV, own0, own1)
     ccd_stats = ctx.ccd_stats() + ctx.ccd_stats_ex() + ctx.ccd_stats_timing()
 
     # ---- per-stage table (CUDA-event pairs around every stage): a separate, eagerly enqueued pass of the same K steps -- event records

@@ -224,6 +224,11 @@ SQUEEZE_OUT_BODIES = [("alien", (0, -1.05, 0), (0, 0, 0), 0.45), ("hollowCat7.5K
                       ("monkey8K", (-0.03, 1.05, 0), (-90, 0, 0), 0.012), ("32770_octocat", (0, 1.9, 0), (-90, 0, 0), 0.01)]
 
 
+def have_squeeze_out_meshes():
+    """the C4 meshes are too large to store in the repository: they exist only where the build cached them (msh.build_asset_cache)"""
+    return all(msh.have_asset(name) for name, *_ in SQUEEZE_OUT_BODIES)
+
+
 def _vertex_normals(V, SF):
     n = np.cross(V[SF[:, 1]] - V[SF[:, 0]], V[SF[:, 2]] - V[SF[:, 0]])
     N = np.zeros_like(V)

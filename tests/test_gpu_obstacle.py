@@ -163,7 +163,6 @@ def test_tail_is_validated(gpu_ctx):
     remove_obstacle(gpu_ctx)
 
 
-@pytest.mark.skipif(not __import__("ipc_b200.msh", fromlist=["msh"]).have_asset("sphere1K"), reason="assets/_ref cache missing")
 def test_c3_ball_over_the_mat_as_obstacle(ctx):
     """BASELINE config C3's bodies with the 200 x 200 mat as the obstacle (80,802 obstacle vertices, 161,600 triangles against sphere1K.msh)"""
     m, info = scenes.ball_on_obstacle_mat(200)

@@ -5,7 +5,7 @@ import pytest
 
 import oracle as orc
 from ipc_b200 import mesh as M
-from ipc_b200 import msh, scenes
+from ipc_b200 import scenes
 
 pytestmark = pytest.mark.gpu
 
@@ -52,20 +52,22 @@ def test_inversion_count_matches_oracle(gpu_ctx):
     assert gpu_ctx.check_inversion() == 0
 
 
-@pytest.mark.skipif(not msh.have_asset("sphere1K"), reason="assets/_ref cache missing")
-def test_full_size_scenes_intersection_counts(gpu_ctx):
+@pytest.mark.parametrize("scene", ["c5", pytest.param("c4", marks=pytest.mark.skipif(
+    not scenes.have_squeeze_out_meshes(), reason="the C4 squeeze-out meshes are too large to store: __graft_entry__.build() caches them where the reference tree is present"))])
+def test_full_size_scenes_intersection_counts(gpu_ctx, scene):
     """C5 (1M tets) is intersection free; C4's manufactured shell crosses its core in places (scenes.squeeze_out_tiled): the device
     must find exactly the triangles the oracle finds, degenerate near-coplanar configurations included."""
     import bench
 
     class A:
-        tets, res, scene = 1_000_000, 10, "c5"
+        tets, res = 1_000_000, 10
 
-    for m in (bench.build_scene(A)[0], scenes.squeeze_out_tiled()[0]):
-        upload(gpu_ctx, m)
-        ok_ref, hits_ref = orc.Surf(m).intersection_free(nthreads=64)
-        gpu_ctx.intersection_free(want=False)
-        gpu_ctx.check_inversion(want=False)
-        it = gpu_ctx.fetch_iteration()
-        assert it.n_intersected_triangles == hits_ref and (hits_ref == 0) == ok_ref
-        assert it.n_inverted_tets == 0
+    A.scene = scene
+    m = bench.build_scene(A)[0] if scene == "c5" else scenes.squeeze_out_tiled()[0]
+    upload(gpu_ctx, m)
+    ok_ref, hits_ref = orc.Surf(m).intersection_free(nthreads=64)
+    gpu_ctx.intersection_free(want=False)
+    gpu_ctx.check_inversion(want=False)
+    it = gpu_ctx.fetch_iteration()
+    assert it.n_intersected_triangles == hits_ref and (hits_ref == 0) == ok_ref
+    assert it.n_inverted_tets == 0
